@@ -430,6 +430,38 @@ def param_tensors(trainer):
     return [p.detach() for p in trainer.parameters()]
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def last_update_outputs(name, trainer, out, batch):
+    """What the last timed update hands its caller, as host arrays named `<name>.<field>`:
+    the loss(es) train_batch returned, the replay indices of the batch it trained on (float64,
+    exact below 2^53), the batch's Q-values where the trainer exposes them, and every parameter
+    after the update."""
+    arrays = {f"{name}.indices": batch.indices.reshape(-1).double()}
+    for i, loss in enumerate(out if isinstance(out, tuple) else (out,)):
+        if loss is not None:
+            arrays[f"{name}.loss{i}"] = loss
+    if getattr(trainer, "all_action_scores", None) is not None:
+        arrays[f"{name}.all_action_scores"] = trainer.all_action_scores
+    for pname, p in trainer.named_parameters():
+        arrays[f"{name}.{pname}"] = p
+    return {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+
+
+def dump_outputs(path, arrays):
+    """Writes every array as `<path>/<name>.npy`."""
+    import numpy as np
+
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed {DUMP_LIMIT_BYTES}")
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (k, a.dtype)
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def dp_check(env, cfg, rb):
     """N > 1: one data-parallel update (row shards, fused gradient exchange) against one
     full-global-batch update on a single rank, from identical parameters and identical draws.
@@ -601,6 +633,11 @@ def run_dqn(env, args, clocks):
     e1.record()
     env.barrier()
     dev_ms = env.max_over_ranks(e0.elapsed_time(e1))
+    outputs = None
+    if args.dump_outputs:
+        # the graph's last update trained on the last batch it keeps; the loss is the
+        # workspace scalar train_batch returns
+        outputs = last_update_outputs("dqn", trainer, trainer._ws["loss"], g_timed._rb200_keep[-1])
 
     # ---- weak scaling (secondary): 4096 rows per rank, rank-specific draws ----
     weak = None
@@ -662,6 +699,8 @@ def run_dqn(env, args, clocks):
     }
     if check:
         res["dp_check"] = check
+    if outputs is not None:
+        res["outputs"] = outputs
     return res
 
 
@@ -676,7 +715,7 @@ def run_generic(env, args, cfg):
     from reagent_b200.replay_memory import PrioritizedReplayBuffer
 
     dev, world, pg = env.dev, env.world, env.pg
-    K = max(3, min(args.steps, {"qrdqn": 20, "sac": 50, "td3": 50}[cfg["algo"]]))
+    K = args.steps
     W = 3
     Bg = cfg["B"]
     lo, hi = env.shard(Bg)
@@ -740,10 +779,12 @@ def run_generic(env, args, cfg):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(K):
-        trainer.train_batch(sample(qs[W + i]), W + i, process_group=pg)
+        batch = sample(qs[W + i])
+        out = trainer.train_batch(batch, W + i, process_group=pg)
     e1.record()
     env.barrier()
     dev_ms = env.max_over_ranks(e0.elapsed_time(e1))
+    outputs = last_update_outputs(cfg["algo"], trainer, out, batch) if args.dump_outputs else None
     kern_ms = None
     if getattr(trainer, "_kernel_events", None):
         durs = [a.elapsed_time(b) for a, b in trainer._kernel_events]
@@ -780,6 +821,8 @@ def run_generic(env, args, cfg):
             "ncu_file": None}
     if check:
         res["dp_check"] = check
+    if outputs is not None:
+        res["outputs"] = outputs
     return res
 
 
@@ -837,6 +880,8 @@ def run_ours(args):
             cpu[c] = {"value": v, "unit": "updates/s", "cores": cores, "kind": "port", "sample": sample}
     if env.rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: v for r in [res] + extra for k, v in r["outputs"].items()})
     peaks = {}
     try:
         with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
@@ -885,7 +930,13 @@ def main():
     ap.add_argument("--only", action="store_true", help="config 2: skip the configs 3-5 array")
     ap.add_argument("--cpu-steps", type=int, default=60)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed update of each config "
+                         "computed (loss, sampled indices, Q-values, parameters) as DIR/<name>.npy; "
+                         "inputs are seeded, so runs with the same arguments are comparable")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:
