@@ -69,7 +69,9 @@ __device__ __forceinline__ float act_bwd_from_out(float y, int act) {
     case RB200_ACT_TANH: return 1.f - y * y;
     case RB200_ACT_LEAKY_RELU: return y > 0.f ? 1.f : 0.01f;
     case RB200_ACT_SIGMOID: return y * (1.f - y);
-    case RB200_ACT_SOFTPLUS: return 1.f - expf(-y);
+    // softplus'(x) = sigmoid(x) = 1 - exp(-y); expm1 keeps it accurate for small y (x << 0),
+    // where 1 - expf(-y) cancels (relative error ~0.5 at x = -16)
+    case RB200_ACT_SOFTPLUS: return -expm1f(-y);
     default: return 1.f;
   }
 }

@@ -18,8 +18,8 @@
 //
 // One CTA = (layer, 128-feature tile of dZ_l, 256-feature tile of A_{l-1}, batch slab); the
 // slabs are summed later by the Adam kernel in slab order (deterministic), exactly like the
-// mma.sync kernel this one replaces for shapes that fit (rb200_optim.cu keeps that kernel for
-// the rest).  Two smem stages; the loads of chunk c+1 are in flight while chunk c's MMAs run.
+// mma.sync kernel in rb200_optim.cu, which stays the default (RB200_WGRAD_TC=1 selects this one
+// for every layer).  Two smem stages; the loads of chunk c+1 are in flight while chunk c's MMAs run.
 #include <stdlib.h>
 
 #include "rb200_umma.cuh"
@@ -261,8 +261,9 @@ __global__ void __launch_bounds__(kWtThreads, 1) wgrad_tc_kernel(const WtParams 
 
 using namespace rb200;
 
-// Launch the tcgen05 weight-gradient kernel.  Returns RB200_E_SMEM when the shapes do not fit
-// (the caller then uses the mma.sync kernel); every layer of the in-scope networks does.
+// Launch the tcgen05 weight-gradient kernel.  Any layer shape fits (128 x 256 feature tiles,
+// 32-row batch chunks, fixed shared-memory size), so there is no shape check here; a launch or
+// opt-in error is returned as is: rb200_mlp_wgrad does not fall back to the mma.sync kernel.
 int rb200_wgrad_tc_launch(const rb200_mlp_t* net, const float* net_input, int32_t batch,
                           const rb200_net_ws_t* ws, float* gpart, int32_t splits, void* stream) {
   WtParams p = {};
